@@ -5,6 +5,7 @@ BM25 top-100 (config C2), at 1/2/4/8 B200.
     python bench.py --gpus N --steps K --warmup W            our CUDA path (torchrun for N>1)
     python bench.py --impl reference --gpus N --steps K ...  the reference's own CPU Enquire::get_mset
     python bench.py --config C3|C5|C4 ...                    the other BASELINE.json configurations (default C2)
+    python bench.py ... --dump-outputs DIR                   also write the last timed step's MSets as DIR/*.npy
 
 A "step" is one pass of the hot path over one batch of BATCH synthetic queries.
   value  — whole-job queries/s with the batch's plan already resident in HBM (device-timed with CUDA
@@ -393,6 +394,39 @@ class CudaArray:
                                          "version": 2}
 
 
+DUMP_LIMIT = 64 << 20
+
+
+def mset_arrays(prefix, n, docids, weights, extra=()):
+    """One timed path's MSets as float64 arrays: [nq, stride] docids and weights (entries past a query's n set
+    to 0, since no docid is 0) plus per-query columns."""
+    import numpy as np
+    n = np.asarray(n, np.int64)
+    keep = np.arange(docids.shape[1])[None, :] < n[:, None]
+    out = {f"{prefix}_n": n.astype(np.float64),
+           f"{prefix}_docids": np.where(keep, docids, 0).astype(np.float64),
+           f"{prefix}_weights": np.where(keep, weights, 0.0).astype(np.float64)}
+    for name, col in extra:
+        out[f"{prefix}_{name}"] = np.asarray(col, np.float64)
+    return out
+
+
+def dump_outputs(path, arrays, suffix=""):
+    """Write DIR/<name><suffix>.npy.  Rows are queries; above DUMP_LIMIT bytes in all, a fixed seeded sample of the
+    rows is written, and query_index.npy says which."""
+    import numpy as np
+    nq = len(next(iter(arrays.values())))
+    row_bytes = sum(a[0].nbytes for a in arrays.values()) + 8
+    budget = DUMP_LIMIT - 4096 * (len(arrays) + 1)  # room for the .npy headers
+    rows = np.arange(nq)
+    if nq * row_bytes > budget:
+        rows = np.sort(np.random.default_rng(0).choice(nq, budget // row_bytes, replace=False))
+    os.makedirs(path, exist_ok=True)
+    np.save(os.path.join(path, f"query_index{suffix}.npy"), rows.astype(np.float64))
+    for name, a in arrays.items():
+        np.save(os.path.join(path, f"{name}{suffix}.npy"), a[rows])
+
+
 def ours(args):
     import numpy as np
     import torch
@@ -606,6 +640,18 @@ def ours(args):
     barrier()
     sampler.end()
     dev_ms = ev0.elapsed_time(ev1)
+    dump = {}
+    if args.dump_outputs:  # what the last replay left on the device: the slab (N = 1) / the merged MSets (N > 1)
+        if world == 1:
+            wp, dp, cp, stride = searchers[0].device_results()
+            w = torch.as_tensor(CudaArray(wp, (BATCH, stride), "<f8"), device="cuda").cpu().numpy()
+            d = torch.as_tensor(CudaArray(dp, (BATCH, stride), "<i4"), device="cuda").cpu().numpy().view(np.uint32)
+            cnt = torch.as_tensor(CudaArray(cp, (BATCH, 8), "<i4"), device="cuda").cpu().numpy().view(np.uint32)
+            dump.update(mset_arrays("replay", cnt[:, 0], d, w, [("exact_matches", cnt[:, 1])]))  # XgmDevResult n, exact
+        else:
+            ow, od, on = xbuf[(args.steps - 1) % 2][6:]
+            dump.update(mset_arrays("replay", on.cpu().numpy(), od.cpu().numpy().view(np.uint32).reshape(QL, TOPK),
+                                    ow.cpu().numpy().reshape(QL, TOPK)))
     # per-launch time of the dominant kernel: K more replays, reading each launch's own events
     for k in range(args.steps):
         searchers[0].replay()
@@ -657,11 +703,26 @@ def ours(args):
         for j in range(max(0, args.steps - LAG), args.steps):
             finish(j)
     for j in range(max(0, args.steps - NSEARCH), args.steps):
-        wait(searchers[j % NSEARCH])
+        last = wait(searchers[j % NSEARCH])
     pending = (args.steps - 1) % NSEARCH
     torch.cuda.synchronize()
     t1 = time.perf_counter()
     sampler.end()
+    if args.dump_outputs:  # the last step's MSets as the caller holds them: scattered by xgm_search_wait / merged
+        if world == 1:
+            l_docids, l_weights, l_keys, l_info = last
+            inf = np.ctypeslib.as_array(l_info)[:BATCH]
+            cols = ["first", "matches_lower_bound", "matches_estimated", "matches_upper_bound", "exact_matches", "status",
+                    "flags", "max_possible", "max_attained", "percent_scale_factor"]
+            if cfg["values"]:
+                keys = np.where(np.arange(TOPK)[None, :] < inf["n"][:, None].astype(np.int64), l_keys.reshape(BATCH, TOPK), 0)
+                cols += [("sort_key_hi", keys >> np.uint64(32)), ("sort_key_lo", keys & np.uint64(0xffffffff))]
+            dump.update(mset_arrays("e2e", inf["n"], l_docids.reshape(BATCH, TOPK), l_weights.reshape(BATCH, TOPK),
+                                    [c if isinstance(c, tuple) else (c, inf[c]) for c in cols]))
+        else:
+            hw, hd, hn = host_out[pending]
+            dump.update(mset_arrays("e2e", hn.numpy(), hd.numpy().view(np.uint32).reshape(QL, TOPK),
+                                    hw.numpy().reshape(QL, TOPK)))
     e2e_s = t1 - t0
     t = torch.tensor([e2e_s], dtype=torch.float64, device="cuda")
     if world > 1:
@@ -756,6 +817,8 @@ def ours(args):
                                     "sample": f"unavailable: {e}"}
     if rank == 0:
         print(json.dumps(line))
+    if dump:
+        dump_outputs(args.dump_outputs, dump, "" if world == 1 else f".rank{rank}")
     if world > 1:
         if shm is not None:
             dist.barrier()
@@ -773,7 +836,11 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-parity", action="store_true", help="skip the dump diff against the compiled reference")
     ap.add_argument("--config", default="C2", choices=sorted(CONFIGS), help="BASELINE.json configuration (default C2)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the MSets of the last timed step of each timed path as DIR/<name>.npy (float64)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     if args.impl == "reference":
         return reference_arm(args)
     return ours(args)

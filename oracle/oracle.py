@@ -27,16 +27,42 @@ SORT_REL, SORT_VAL_REL, SORT_VAL, SORT_REL_VAL = 0, 1, 2, 3
 FILTER_NONE, FILTER_VALUE_RANGE_MIN, FILTER_MULTI_RANGE = 0, 1, 2
 
 
+def _digest(deps: Sequence[str], recipe: Sequence[str]) -> str:
+    import hashlib
+    repo = os.path.dirname(HERE)  # the command names paths inside the tree; where the tree lies does not count
+    h = hashlib.sha256("\0".join(recipe).replace(repo, "").encode())
+    for d in deps:
+        with open(d, "rb") as f:
+            h.update(hashlib.sha256(f.read()).digest())
+    return h.hexdigest()
+
+
+def stale(target: str, deps: Sequence[str], recipe: Sequence[str]) -> bool:
+    """True unless target exists and target.sha256 holds the digest of the contents of deps and of the build
+    command it was made from.  Contents, not modification times: a tree that was copied or checked out again
+    keeps its build products, while a changed source or flag still rebuilds."""
+    try:
+        with open(target + ".sha256") as f:
+            return not os.path.exists(target) or f.read().strip() != _digest(deps, recipe)
+    except OSError:
+        return True
+
+
+def mark_built(target: str, deps: Sequence[str], recipe: Sequence[str]) -> None:
+    with open(target + ".sha256", "w") as f:
+        f.write(_digest(deps, recipe) + "\n")
+
+
 def build(force: bool = False) -> str:
     """Compile the C restatement (gcc, no FMA contraction)."""
     src = os.path.join(HERE, "xgm_oracle.c")
     deps = [src, os.path.join(HERE, "xgm_oracle.h"),
             os.path.join(HERE, "..", "xapiand_b200", "csrc", "xgm_corpus.h")]
-    if (not force and os.path.exists(LIB_PATH)
-            and all(os.path.getmtime(LIB_PATH) >= os.path.getmtime(d) for d in deps)):
+    cmd = ["gcc", "-O2", "-ffp-contract=off", "-fPIC", "-shared", "-Wall", "-o", LIB_PATH, src, "-lm"]
+    if not force and not stale(LIB_PATH, deps, cmd):
         return LIB_PATH
-    subprocess.check_call(["gcc", "-O2", "-ffp-contract=off", "-fPIC", "-shared", "-Wall",
-                           "-o", LIB_PATH, src, "-lm"])
+    subprocess.check_call(cmd)
+    mark_built(LIB_PATH, deps, cmd)
     return LIB_PATH
 
 

@@ -63,21 +63,24 @@ def run_set(tag, ndocs, vocab, queries, nshards=1, twophase=False, values=False,
         shutil.rmtree(tmp, ignore_errors=True)
 
 
-def run_mv_set(tag, ndocs, vocab, queries, sparse=(7, 5), seed=12345):
+def run_mv_set(tag, ndocs, vocab, queries, sparse=(7, 5), seed=12345, db=None, with_slots=True):
     """Xapiand's own multivalue classes (oracle/_ref/libxapiand_mv_ref.so = src/multivalue/range.cc, keymaker.cc …
     compiled from the reference): slots written as StringLists of Serialise::positive keys, MultipleValueRange as
-    OP_FILTER right side or weighted OP_AND child, Multi_MultiValueKeyMaker{SerialiseKey} as the sorter."""
+    OP_FILTER right side or weighted OP_AND child, Multi_MultiValueKeyMaker{SerialiseKey} as the sorter.
+    db: an existing database of that corpus to query instead of building one; with_slots=False leaves the
+    per-document slot bytes out of the fixture (a test that opens the database itself does not need them)."""
     import subprocess
     tmp = tempfile.mkdtemp(prefix="xgm_golden_")
     try:
-        d = os.path.join(tmp, "db")
-        O.ref_build(d, ndocs, vocab, seed=seed, mvalues=True, sparse=sparse)
+        d = db or os.path.join(tmp, "db")
+        if db is None:
+            O.ref_build(d, ndocs, vocab, seed=seed, mvalues=True, sparse=sparse)
         lines = [O.query_line("TERM" if len(q["terms"]) == 1 else "AND", [name(t) for t in q["terms"]], q["first"],
                               q["maxitems"], q["check_at_least"], mvr=q.get("mvr"), keysort=q.get("keysort"))
                  for q in queries]
         info, res = O.ref_query([d], lines, os.path.join(tmp, "w"))
         slots = {}
-        for ln in subprocess.check_output([O.REF_RUNNER, "slots", "--db", d]).decode().splitlines():
+        for ln in subprocess.check_output([O.REF_RUNNER, "slots", "--db", d]).decode().splitlines() if with_slots else []:
             sl, did, hx = (ln.split() + [""])[:3]
             slots.setdefault(sl, {})[did] = hx
         nums = sorted({v for q in queries if q.get("mvr") for v in q["mvr"][1:3]})
@@ -97,6 +100,91 @@ def run_mv_set(tag, ndocs, vocab, queries, sparse=(7, 5), seed=12345):
         with open(os.path.join(OUT, f"{tag}.json"), "w") as f:
             json.dump(fixture, f, separators=(",", ":"))
         print(tag, len(queries), "queries", os.path.getsize(os.path.join(OUT, f"{tag}.json")), "bytes")
+    finally:
+        shutil.rmtree(tmp, ignore_errors=True)
+
+
+#        name                    docs  vocab  seed   ref_build options
+GLASS = [("plain_1k",             1000, 300,   5,     {}),
+         ("mvalues_sparse_1500",  1500, 600,   12345, dict(mvalues=True, sparse=[7, 5])),
+         ("values_2k",            2000, 40,    5,     dict(values=True)),
+         ("single_doc",           1,    5,     5,     {})]
+
+
+def _export_digest(db, flat):
+    """Size and SHA-256 of the flat file `ref_runner export` writes by walking db through the public iterators."""
+    import hashlib
+    import subprocess
+    subprocess.check_call([O.REF_RUNNER, "export", "--db", db, "--out", flat], stdout=subprocess.DEVNULL)
+    data = open(flat, "rb").read()
+    return len(data), hashlib.sha256(data).hexdigest()
+
+
+def _tar_xz(src_dir, dst):
+    """The database directory as a reproducible .tar.xz (sorted members, no owner or time stamps)."""
+    import lzma
+    import tarfile
+    with lzma.open(dst, "wb", preset=9 | lzma.PRESET_EXTREME) as xz, tarfile.open(fileobj=xz, mode="w") as tar:
+        for fn in sorted(os.listdir(src_dir)):
+            ti = tar.gettarinfo(os.path.join(src_dir, fn), arcname=fn)
+            ti.mtime, ti.uid, ti.gid, ti.uname, ti.gname, ti.mode = 0, 0, 0, "", "", 0o644
+            with open(os.path.join(src_dir, fn), "rb") as f:
+                tar.addfile(ti, f)
+
+
+def edge_glass_queries(rng, n, topranks, ndocs):
+    """AND / OR of 1-5 terms, top-10 or top-100, with and without check_at_least = every document."""
+    qs = []
+    for i in range(n):
+        op = "AND" if i % 2 == 0 else "OR"
+        terms = rng.sample(range(topranks), rng.choice([1, 2, 3, 5]))
+        qs.append(dict(op=op, terms=terms, first=0, maxitems=rng.choice([10, 100]), check_at_least=rng.choice([0, ndocs])))
+    return qs
+
+
+def run_glass_sets():
+    """Glass databases written by the reference, for the tests of the direct glass reader (tests/golden/glass/):
+    each database as .tar.xz plus the digest of the reference's own flat export of it (databases.json), the
+    reference's MSets on the multivalue database (multivalue_1500.json), and glass_6k.json: the digest of the
+    export of a 6000-document database and the reference's MSets on it (weights as the SHA-256 of their
+    little-endian float64 bytes, to keep the fixture small)."""
+    import hashlib
+    import numpy as np
+    gdir = os.path.join(OUT, "glass")
+    os.makedirs(gdir, exist_ok=True)
+    tmp = tempfile.mkdtemp(prefix="xgm_golden_")
+    try:
+        meta = {}
+        for tag, ndocs, vocab, seed, kw in GLASS:
+            d = os.path.join(tmp, tag)
+            O.ref_build(d, ndocs, vocab, seed=seed, **kw)
+            size, sha = _export_digest(d, d + ".flat")
+            meta[tag] = dict(ndocs=ndocs, vocab=vocab, seed=seed, **kw, export_bytes=size, export_sha256=sha)
+            _tar_xz(d, os.path.join(gdir, f"{tag}.tar.xz"))
+            print(tag, os.path.getsize(os.path.join(gdir, f"{tag}.tar.xz")), "bytes")
+        with open(os.path.join(gdir, "databases.json"), "w") as f:
+            json.dump(meta, f, indent=1)
+        mv = meta["mvalues_sparse_1500"]
+        run_mv_set("multivalue_1500", mv["ndocs"], mv["vocab"], mv_queries(random.Random(20261017), 80, 60, mv["ndocs"]),
+                   sparse=mv["sparse"], seed=mv["seed"], db=os.path.join(tmp, "mvalues_sparse_1500"), with_slots=False)
+
+        ndocs, vocab, seed = 6000, 800, 99
+        d = os.path.join(tmp, "edge")
+        O.ref_build(d, ndocs, vocab, seed=seed)
+        size, sha = _export_digest(d, d + ".flat")
+        queries = edge_glass_queries(random.Random(12), 80, 120, ndocs)
+        lines = [O.query_line("TERM" if len(q["terms"]) == 1 else q["op"], [name(t) for t in q["terms"]], 0, q["maxitems"],
+                              q["check_at_least"]) for q in queries]
+        _, res = O.ref_query([d], lines, os.path.join(tmp, "w"))
+        for q, r in zip(queries, res):
+            q.update(docids=r.docids, weights_sha256=hashlib.sha256(np.asarray(r.weights, "<f8").tobytes()).hexdigest(),
+                     lb=r.lb, est=r.est, ub=r.ub, max_possible=float(r.max_possible).hex(),
+                     max_attained=float(r.max_attained).hex())
+        fixture = dict(tag="glass_6k", ndocs=ndocs, vocab=vocab, seed=seed, export_bytes=size, export_sha256=sha,
+                       queries=queries)
+        with open(os.path.join(OUT, "glass_6k.json"), "w") as f:
+            json.dump(fixture, f, separators=(",", ":"))
+        print("glass_6k", os.path.getsize(os.path.join(OUT, "glass_6k.json")), "bytes")
     finally:
         shutil.rmtree(tmp, ignore_errors=True)
 
@@ -236,6 +324,9 @@ def bm25_queries(rng, n, topranks, ndocs):
 def main():
     if not O.have_reference():
         raise SystemExit("oracle/_ref not built: run oracle/build_ref.sh (needs /root/reference)")
+    if sys.argv[1:] == ["glass"]:
+        run_glass_sets()
+        return
     if sys.argv[1:] == ["mv"]:
         run_mv_set("multivalue_5k", 5000, 2000, mv_queries(random.Random(20260930), 240, 60, 5000))
         return
@@ -283,6 +374,7 @@ def main():
     run_set("bm25_6k", 6000, 900, bm25_queries(random.Random(20260929), 200, 150, 6000), seed=11)
     run_mv_set("multivalue_5k", 5000, 2000, mv_queries(random.Random(20260930), 240, 60, 5000))
     run_set("orops_6k", 6000, 900, orops_queries(random.Random(20260931), 240, 120, 6000), seed=11)
+    run_glass_sets()
 
 
 if __name__ == "__main__":

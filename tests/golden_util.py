@@ -15,6 +15,21 @@ def load(tag):
     return fx
 
 
+def glass_databases():
+    """tests/golden/glass/databases.json: how each stored database was built and the size and SHA-256 of the flat
+    file the reference's `ref_runner export` wrote from it."""
+    with open(os.path.join(GOLDEN, "glass", "databases.json")) as f:
+        return json.load(f)
+
+
+def glass_db(tag, dest):
+    """Unpack the glass database the reference wrote (tests/golden/glass/<tag>.tar.xz) into dest; returns dest."""
+    import tarfile
+    with tarfile.open(os.path.join(GOLDEN, "glass", f"{tag}.tar.xz")) as tar:
+        tar.extractall(dest, filter="data")
+    return dest
+
+
 def sortable_key_to_int(hexkey: str) -> int:
     """Invert Xapian::sortable_serialise for the non-negative integers the fixtures use.
     Positive x = m * 2^e is stored as 0b11 [large-exponent bit, 3-bit or 10-bit exponent] mantissa..

@@ -1,38 +1,32 @@
 """CPU tests of the direct glass reader (xapiand_b200/csrc/xgm_glass.cu): `xgm_glass_export_flat` parses
 iamglass + postlist.glass itself and must produce, byte for byte, the file `ref_runner export` writes by walking
-the same database through the reference's public iterators (allterms / postlist / doclength / valuestream)."""
-import filecmp
-import os
-import shutil
-import subprocess
-import tempfile
+the same database through the reference's public iterators (allterms / postlist / doclength / valuestream).
+The databases were written by the reference (tests/golden/glass/); the size and SHA-256 of the reference's export
+of each are stored next to them (tests/golden/make_golden.py glass)."""
 import ctypes
+import hashlib
 
 import pytest
 
-from oracle import oracle as O
+from tests.golden_util import glass_databases, glass_db
 from xapiand_b200 import xgm
 
-pytestmark = pytest.mark.skipif(not O.have_reference(), reason="compiled reference (oracle/_ref) not built")
+DATABASES = glass_databases()
 
 
-@pytest.mark.parametrize("ndocs,vocab,kw", [(3000, 500, {}), (20000, 3000, dict(mvalues=True, sparse=(7, 5))),
-                                            (40000, 200, dict(values=True)), (1, 5, {})])
-def test_direct_reader_equals_the_reference_iterators(ndocs, vocab, kw):
-    tmp = tempfile.mkdtemp(prefix="xgm_glass_")
-    try:
-        db = os.path.join(tmp, "db")
-        O.ref_build(db, ndocs, vocab, seed=5, **kw)
-        subprocess.check_call([O.REF_RUNNER, "export", "--db", db, "--out", os.path.join(tmp, "ref.flat")],
-                              stdout=subprocess.DEVNULL)
-        st = xgm.lib().xgm_glass_export_flat(db.encode(), os.path.join(tmp, "mine.flat").encode())
-        assert st == 0, xgm.lib().xgm_last_error()
-        assert filecmp.cmp(os.path.join(tmp, "ref.flat"), os.path.join(tmp, "mine.flat"), shallow=False)
-        rev, dc, last = ctypes.c_uint64(), ctypes.c_uint32(), ctypes.c_uint32()
-        assert xgm.lib().xgm_glass_revision(db.encode(), ctypes.byref(rev), ctypes.byref(dc), ctypes.byref(last)) == 0
-        assert (dc.value, last.value) == (ndocs, ndocs) and rev.value >= 1
-    finally:
-        shutil.rmtree(tmp, ignore_errors=True)
+@pytest.mark.parametrize("tag", sorted(DATABASES))
+def test_direct_reader_equals_the_reference_iterators(tag, tmp_path):
+    ref = DATABASES[tag]
+    db = glass_db(tag, str(tmp_path / "db"))
+    mine = tmp_path / "mine.flat"
+    st = xgm.lib().xgm_glass_export_flat(db.encode(), str(mine).encode())
+    assert st == 0, xgm.lib().xgm_last_error()
+    data = mine.read_bytes()
+    assert (len(data), hashlib.sha256(data).hexdigest()) == (ref["export_bytes"], ref["export_sha256"]), \
+        "the export differs from the reference's"
+    rev, dc, last = ctypes.c_uint64(), ctypes.c_uint32(), ctypes.c_uint32()
+    assert xgm.lib().xgm_glass_revision(db.encode(), ctypes.byref(rev), ctypes.byref(dc), ctypes.byref(last)) == 0
+    assert (dc.value, last.value) == (ref["ndocs"], ref["ndocs"]) and rev.value >= 1
 
 
 def test_reader_rejects_what_is_not_a_glass_database(tmp_path):

@@ -134,41 +134,40 @@ def test_unsupported_shapes_are_declined_not_guessed(edge):
     assert r.status == xgm.E_UNIMPLEMENTED
 
 
-@pytest.mark.skipif(not O.have_reference(), reason="compiled reference (oracle/_ref) not shipped")
 def test_glass_db_through_public_iterators_matches_reference():
     """Drop-in data path: a glass DB written by the reference → `ref_runner export` (Database::allterms_begin /
     postlist_begin / get_doclength, INTEGRATION.md §1) → xgm_index_load_flat → same MSets as the
-    reference's Enquire::get_mset on that very DB."""
-    import subprocess
+    reference's Enquire::get_mset on that very DB (tests/golden/glass_6k.json).  The export is the flat file of
+    the seeded corpus the DB was built from; it is rewritten here and must match the reference's export (size
+    and SHA-256) before it is loaded."""
+    import hashlib
+    import json
+    from tests.golden_util import GOLDEN
+    with open(os.path.join(GOLDEN, "glass_6k.json")) as f:
+        fx = json.load(f)
+    orc = O.Index.synthetic(fx["ndocs"], fx["vocab"], seed=fx["seed"])
     tmp = tempfile.mkdtemp(prefix="xgm_glass_")
     try:
-        db = os.path.join(tmp, "db")
-        O.ref_build(db, 6000, 800, seed=99)
         flat = os.path.join(tmp, "db.flat")
-        subprocess.check_call([O.REF_RUNNER, "export", "--db", db, "--out", flat], stdout=subprocess.DEVNULL)
+        write_flat(flat, orc.doclen(), [(orc.name(t),) + tuple(orc.postings(t)) for t in range(orc.nterms)])
+        data = open(flat, "rb").read()
+        assert (len(data), hashlib.sha256(data).hexdigest()) == (fx["export_bytes"], fx["export_sha256"])
         ix = xgm.Index.load_flat(flat)
-        rng = random.Random(12)
-        qs, lines = [], []
-        for i in range(80):
-            op = "AND" if i % 2 == 0 else "OR"
-            terms = [f"T{r:06d}" for r in rng.sample(range(120), rng.choice([1, 2, 3, 5]))]
-            mi = rng.choice([10, 100])
-            cal = rng.choice([0, 6000])
-            qs.append(xgm.Query(xgm.OP_AND if op == "AND" else xgm.OP_OR, terms, maxitems=mi, check_at_least=cal))
-            lines.append(O.query_line("TERM" if len(terms) == 1 else op, terms, 0, mi, cal))
-        _, ref = O.ref_query([db], lines, os.path.join(tmp, "w"))
-        s = xgm.Searcher(ix, max_batch=len(qs), max_topk=128)
-        for i, (m, r) in enumerate(zip(s.search(qs), ref)):
-            assert m.status == 0
-            assert list(m.docids) == r.docids, f"glass[{i}] {lines[i]}"
-            assert [float(x).hex() for x in m.weights] == [float(x).hex() for x in r.weights], f"glass[{i}]"
-            assert float(m.max_possible).hex() == float(r.max_possible).hex()
-            assert float(m.max_attained).hex() == float(r.max_attained).hex()
-            assert m.matches_upper_bound == r.ub
-            if not (m.flags & 1):
-                assert (m.matches_lower_bound, m.get_matches_estimated()) == (r.lb, r.est), f"glass[{i}] {lines[i]}"
     finally:
         shutil.rmtree(tmp, ignore_errors=True)
+    qs = [xgm.Query(xgm.OP_AND if q["op"] == "AND" else xgm.OP_OR, [f"T{r:06d}" for r in q["terms"]],
+                    maxitems=q["maxitems"], check_at_least=q["check_at_least"]) for q in fx["queries"]]
+    s = xgm.Searcher(ix, max_batch=len(qs), max_topk=128)
+    for i, (m, r) in enumerate(zip(s.search(qs), fx["queries"])):
+        ctx = f"glass[{i}] {r['op']} {r['terms']} maxitems={r['maxitems']} check_at_least={r['check_at_least']}"
+        assert m.status == 0
+        assert list(m.docids) == r["docids"], ctx
+        assert hashlib.sha256(np.asarray(m.weights, "<f8").tobytes()).hexdigest() == r["weights_sha256"], f"{ctx}: weights"
+        assert float(m.max_possible).hex() == r["max_possible"]
+        assert float(m.max_attained).hex() == r["max_attained"]
+        assert m.matches_upper_bound == r["ub"]
+        if not (m.flags & 1):
+            assert (m.matches_lower_bound, m.get_matches_estimated()) == (r["lb"], r["est"]), ctx
 
 
 def test_background_submit_matches_synchronous(edge):

@@ -341,18 +341,18 @@ def test_cuda_matches_xapiand_multivalue_classes():
 def test_direct_glass_reader_index_matches_xapiand_multivalue_classes():
     """SURVEY.md section 8(b) / (f)-3: xgm_index_open reads the glass directory itself (iamglass + the postlist B-tree:
     posting chunks, document lengths, value streams) — the same fixture as above must come out of an index built that
-    way from the database the reference wrote, carrying the database's own revision."""
+    way from the database the reference wrote, carrying the database's own revision.  The database is
+    tests/golden/glass/mvalues_sparse_1500.tar.xz, the reference's MSets on it multivalue_1500.json."""
     import ctypes
     import shutil
     import tempfile
-    from oracle import oracle as O
-    if not O.have_reference():
-        pytest.skip("compiled reference (oracle/_ref) not shipped")
-    fx = load("multivalue_5k")
+    from tests.golden_util import glass_databases, glass_db
+    fx = load("multivalue_1500")
+    built = glass_databases()["mvalues_sparse_1500"]
+    assert (built["ndocs"], built["vocab"], built["seed"], built["sparse"]) == (fx["ndocs"], fx["vocab"], fx["seed"], fx["sparse"])
     tmp = tempfile.mkdtemp(prefix="xgm_glass_")
     try:
-        db = tmp + "/db"
-        O.ref_build(db, fx["ndocs"], fx["vocab"], seed=fx["seed"], mvalues=True, sparse=fx["sparse"])
+        db = glass_db("mvalues_sparse_1500", tmp + "/db")
         rev = ctypes.c_uint64()
         assert xgm.lib().xgm_glass_revision(db.encode(), ctypes.byref(rev), None, None) == 0
         ix = xgm.Index.open_glass(db)
